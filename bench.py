@@ -430,6 +430,29 @@ def parity_check(args, alg, A, B, Sv, res, rank, world, pattern_ref, want_full):
     return out
 
 
+DUMP_SEED = 20261017
+DUMP_BYTES = 64_000_000   # every file of every rank together, headers included
+
+
+def dump_outputs(out_dir, A, values, rank, world):
+    """What the last timed fusedSpMM returned to this rank's caller -- A (the FusedMM output, mode A) and the SDDMM
+    values -- as float64 .npy files under `out_dir`.  Each rank gets an equal share of DUMP_BYTES, two thirds for A
+    and one third for the values; an output larger than its share is cut to a fixed seeded sample of rows / values
+    (sorted indices, identical for identical arguments), so two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    share = DUMP_BYTES // world - 2 * 128  # an .npy header is 128 bytes
+    row_bytes = 8 * max(1, A.shape[1])
+    rows, nvals = min(A.shape[0], (2 * share // 3) // row_bytes), min(values.size, (share // 3) // 8)
+    rng = np.random.default_rng(DUMP_SEED)
+    if rows < A.shape[0]:
+        A = A[np.sort(rng.choice(A.shape[0], rows, replace=False))]
+    if nvals < values.size:
+        values = values[np.sort(rng.choice(values.size, nvals, replace=False))]
+    np.save(os.path.join(out_dir, f"fused_output_A{suffix}.npy"), np.ascontiguousarray(A, np.float64))
+    np.save(os.path.join(out_dir, f"sddmm_values{suffix}.npy"), np.ascontiguousarray(values, np.float64))
+
+
 # ------------------------------------------------------------------ GPU arm ---------------
 def run_native(args):
     import torch
@@ -498,6 +521,8 @@ def run_native(args):
     sync_barrier()
     launches = L.hnh_launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs:  # before the legs below overwrite A
+        dump_outputs(args.dump_outputs, A.to_host(), res.to_host(), rank, world)
     ms = max_over_ranks(ms_total) / args.steps
     flops = 4.0 * nnz * R
     gflops = flops / (ms * 1e-3) / 1e9
@@ -678,7 +703,14 @@ def main():
                     help="correctness leg after the timed loops (never timed): 'sample' = a row sample per rank against the "
                          "C port of the reference kernels; 'full' = that plus every output row against one fusedSpMM of "
                          "oracle/_ref (the reference's own code) on the same tuples and operands")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="native arm: write what the last timed step computed (A and the SDDMM values, or a fixed "
+                         "sample of them) as DIR/<name>.npy, float64, at most 64 MB over all ranks")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes what the native (GPU) arm computed; the reference arm has nothing to dump")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.c <= 0:
         args.c = default_c(args.alg, world)

@@ -8,6 +8,8 @@ import tempfile
 
 import numpy as np
 
+from tests import golden_util as G
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ALL_OPS = ["sddmmA", "spmmA", "spmmB", "fusedA", "sddmmB", "fusedB"]
 
@@ -72,32 +74,59 @@ def reference_for(case_, p):
     return None, None
 
 
-def flatten_ref(ranks):
-    """ref.run output -> flat dict of arrays (the golden-file format)."""
+WRITE_GOLDEN = False  # set by scripts/make_golden.py: reference_arrays also stores what it computed
+
+
+def reference_arrays(name, compute, exact=()):
+    """A dict of reference arrays: `compute()` where oracle/_ref is built, else tests/golden/<name>.npz (written from
+    the same `compute` by scripts/make_golden.py; the keys in `exact` are compared bit for bit, the others within a
+    tolerance).  Returns (arrays, source)."""
+    from oracle import ref
+    path = os.path.join(ROOT, "tests", "golden", f"{name}.npz")
+    if ref.available():
+        arrays = compute()
+        if WRITE_GOLDEN:
+            out = {}
+            for k, a in arrays.items():
+                G.reduce_into(out, k, a, k in exact)
+            G.save(path, out)
+        return arrays, "oracle/_ref"
+    z = G.open_golden(path)
+    return {k: G.load(z, k) for k in {f.split("__")[0] for f in z.files}}, "tests/golden"
+
+
+def flatten_ref(ranks, reduced=False, alg=None):
+    """ref.run output -> flat dict of arrays (the golden-file format).  reduced: large arrays in the reduced form of
+    tests/golden_util.py (layout: digests; operation outputs: sample + sketch)."""
     flat = {}
+    put = (lambda k, a, exact: G.reduce_into(flat, k, a, exact)) if reduced else (lambda k, a, exact: flat.update({k: a}))
     for r, d in enumerate(ranks):
         for k in ("i", "j", "k", "localArows", "localAcols", "localBrows", "localBcols"):
             flat[f"r{r}_{k}"] = np.int64(d[k])
         for k in ("aSubmatrices", "bSubmatrices", "S_rows", "S_cols", "ST_rows", "ST_cols"):
-            flat[f"r{r}_{k}"] = d[k]
+            put(f"r{r}_{k}", d[k], True)
         for key in ("S", "ST"):
             flat[f"r{r}_{key}_nblocks"] = np.int64(len(d[key + "_blocks"]))
             for b, blk in enumerate(d[key + "_blocks"]):
                 flat[f"r{r}_{key}_b{b}_null"] = np.bool_(blk is None)
                 if blk is not None:
+                    blk = dict(blk)
+                    if reduced and alg == "25d_dense_replicate":  # see compare_layout: what this library must hold
+                        blk["row_idx"] = np.repeat(np.arange(int(blk["rows"])), np.diff(np.asarray(blk["rowStart"])))
                     for f in ("rows", "cols", "transpose", "rowStart", "col_idx", "row_idx", "values"):
-                        flat[f"r{r}_{key}_b{b}_{f}"] = np.asarray(blk[f])
+                        put(f"r{r}_{key}_b{b}_{f}", np.asarray(blk[f]), True)
         flat[f"r{r}_nops"] = np.int64(len(d["ops"]))
         for t, op in enumerate(d["ops"]):
-            flat[f"r{r}_op{t}_A"], flat[f"r{r}_op{t}_B"], flat[f"r{r}_op{t}_values"] = op["A"], op["B"], op["values"]
+            for f in ("A", "B", "values"):
+                put(f"r{r}_op{t}_{f}", op[f], False)
     return flat
 
 
 def load_golden(path, p):
-    z = np.load(path, allow_pickle=False)
+    z = G.open_golden(path)
     ranks = []
     for r in range(p):
-        g = lambda k: z[f"r{r}_{k}"]
+        g = lambda k: G.load(z, f"r{r}_{k}")  # noqa: E731
         d = {k: int(g(k)) for k in ("i", "j", "k", "localArows", "localAcols", "localBrows", "localBcols")}
         for k in ("aSubmatrices", "bSubmatrices", "S_rows", "S_cols", "ST_rows", "ST_cols"):
             d[k] = g(k)
@@ -119,8 +148,8 @@ def compare_layout(got, want, alg):
     for r, (g, w) in enumerate(zip(got, want)):
         for k in ("i", "j", "k", "localArows", "localAcols", "localBrows", "localBcols"):
             assert int(g[k]) == int(w[k]), (r, k, int(g[k]), int(w[k]))
-        assert np.array_equal(g["aSubmatrices"], w["aSubmatrices"]), (r, "aSubmatrices")
-        assert np.array_equal(g["bSubmatrices"], w["bSubmatrices"]), (r, "bSubmatrices")
+        assert G.same(g["aSubmatrices"], w["aSubmatrices"]), (r, "aSubmatrices")
+        assert G.same(g["bSubmatrices"], w["bSubmatrices"]), (r, "bSubmatrices")
         for key in ("S", "ST"):
             wb = w[key + "_blocks"]
             assert int(g[key + "_nblocks"]) == len(wb), (r, key, "block count")
@@ -137,15 +166,18 @@ def compare_layout(got, want, alg):
                     assert len(g[f"{key}_b{b}_col_idx"]) == 0 and not np.any(g[f"{key}_b{b}_rowStart"]), (r, key, b, "empty block")
                     continue
                 for f in ("rowStart", "col_idx", "row_idx", "values"):
-                    have, ref_ = np.asarray(g[f"{key}_b{b}_{f}"]), np.asarray(blk[f])
-                    if f == "row_idx" and alg == "25d_dense_replicate" and not np.array_equal(have, ref_):
+                    have, ref_ = np.asarray(g[f"{key}_b{b}_{f}"]), blk[f]
+                    if (f == "row_idx" and alg == "25d_dense_replicate" and not G.same(have, ref_)
+                            and not isinstance(blk["rowStart"], G.Reduced)):
                         # The reference's setup skew ships the block in `both` mode and never waits for the row_idx
                         # receive (`else if`, SpmatLocal.hpp:248-255; SURVEY.md appendix B.2): whether its row_idx has
                         # landed when the block is dumped is a race in the reference itself (seen on a 128-core box).
                         # rowStart and col_idx (waited for, compared above) define the block; the delivered row_idx is
                         # their expansion, which is what this library must hold.
                         ref_ = np.repeat(np.arange(int(blk["rows"])), np.diff(np.asarray(blk["rowStart"])))
-                    if not np.array_equal(have, ref_):
+                    if not G.same(have, ref_):
+                        if isinstance(ref_, G.Reduced):  # stored as a digest: no entries to show
+                            raise AssertionError((r, key, b, f, f"shape {have.shape}", f"differs from {ref_}"))
                         where = np.flatnonzero(have != ref_)[:6] if have.shape == ref_.shape else []
                         raise AssertionError((r, key, b, f, f"shapes {have.shape} {ref_.shape}", f"first diffs at {list(where)}",
                                               f"have {have[where].tolist() if len(where) else ''}",
@@ -156,13 +188,13 @@ def compare_ops(got, want, script, rtol=1e-11):
     worst = 0.0
     for r, (g, w) in enumerate(zip(got, want)):
         for key in ("S_rows", "S_cols", "ST_rows", "ST_cols"):
-            assert np.array_equal(g[key], w[key]), (r, key)  # order of the local value vectors: bit-exact
+            assert G.same(g[key], w[key]), (r, key)  # order of the local value vectors: bit-exact
         for t, op in enumerate(script):
             for f in ("A", "B", "values"):
                 a, b = g[f"op{t}_{f}"], w["ops"][t][f]
-                assert a.shape == b.shape, (r, op, f, a.shape, b.shape)
+                assert a.shape == tuple(b.shape), (r, op, f, a.shape, b.shape)
                 if a.size:
-                    err = np.abs(a - b).max() / max(np.abs(b).max(), 1e-300)
+                    err = G.rel_err(a, b)
                     worst = max(worst, err)
                     assert err < rtol, (r, op, f, err)
     return worst

@@ -229,22 +229,33 @@ def test_p1_gat_forward_matches_global_model(world, name):
 
 @pytest.mark.parametrize("name", ALGS)
 def test_p1_als_cg_matches_reference_als(world, name):
-    """One alternating round of batched CG on given inputs against the reference's own Distributed_ALS (oracle/_ref)."""
-    from oracle import ref
+    """One alternating round of batched CG on given inputs against the reference's own Distributed_ALS (oracle/_ref, or
+    its golden file)."""
+    from tests import golden_util as G
     from tests.mp_worker import als_inputs
-    if not ref.available():
-        pytest.skip("oracle/_ref is not built")
     logM, npr, R = 8, 6, 16
     N = 1 << logM
-    rows, cols, _ = orc.er_tuples(logM, npr, SEED)
     Agt, Bgt, A0, B0 = als_inputs(N, R, SEED)
     S = D.SpmatLocal.load_er(logM, npr, SEED)
     alg = D.Algorithm(name, S, R, 1)
     res, A, B = D.als_run(alg, Agt, Bgt, A0, B0, 1, 10)
-    want = ref.als(name, 1, 1, R, N, rows, cols, Agt, Bgt, A0, B0, 1, 10)
+    want, _ = p1_als_reference(name)
     assert res[1] < 0.5 * res[0]
     assert np.allclose(res, want["residual"], rtol=1e-7, atol=0)
-    assert rel_err(A, want["A"]) < 1e-7 and rel_err(B, want["B"]) < 1e-7
+    assert G.rel_err(A, want["A"]) < 1e-7 and G.rel_err(B, want["B"]) < 1e-7
+
+
+def p1_als_reference(name):
+    def compute():
+        from oracle import ref
+        from tests.mp_worker import als_inputs
+        logM, npr, R = 8, 6, 16
+        N = 1 << logM
+        rows, cols, _ = orc.er_tuples(logM, npr, SEED)
+        want = ref.als(name, 1, 1, R, N, rows, cols, *als_inputs(N, R, SEED), 1, 10)
+        return {"residual": np.asarray(want["residual"]), "A": want["A"], "B": want["B"]}
+    from tests import mp_util as U
+    return U.reference_arrays(f"als_p1_{name}", compute)
 
 
 @pytest.mark.parametrize("R", [12, 192])

@@ -18,11 +18,11 @@ CASES_2 = [
     U.case("15d_fusion2", 1, 8, 7, 5, n=101),
     U.case("15d_sparse", 1, 8, 7, 5, n=101),
     # rectangular matrices (more columns than rows and the reverse; neither divides evenly)
-    U.case("15d_fusion2", 1, 8, 7, 5, n=120, m=75, name="nogolden_rect_fusion2"),
-    U.case("15d_sparse", 2, 8, 7, 5, n=70, m=128, name="nogolden_rect_sparse"),
-    # 650k tuples: the multi-threaded bucketing / counting-sort paths of the setup (needs oracle/_ref; no golden file)
-    U.case("15d_fusion1", 1, 8, 14, 40, name="nogolden_big_fusion1"),
-    U.case("25d_sparse_replicate", 2, 8, 14, 40, name="nogolden_big_25d_sparse"),
+    U.case("15d_fusion2", 1, 8, 7, 5, n=120, m=75, name="rect_fusion2"),
+    U.case("15d_sparse", 2, 8, 7, 5, n=70, m=128, name="rect_sparse"),
+    # 650k tuples: the multi-threaded bucketing / counting-sort paths of the setup
+    U.case("15d_fusion1", 1, 8, 14, 40, name="big_fusion1"),
+    U.case("25d_sparse_replicate", 2, 8, 14, 40, name="big_25d_sparse"),
 ]
 CASES_4 = [
     U.case("15d_fusion1", 2, 8, 7, 5),
@@ -32,17 +32,17 @@ CASES_4 = [
     U.case("15d_fusion1", 2, 8, 7, 5, n=99),
     U.case("25d_dense_replicate", 1, 8, 7, 5, n=99),
     # any initial distribution of the tuples is legal input: all on the last rank / scattered and handed over unsorted
-    dict(U.case("15d_fusion2", 2, 8, 7, 5, n=101, m=90, name="nogolden_deal_last"), deal="last"),
-    dict(U.case("15d_sparse", 1, 8, 7, 5, n=101, m=90, name="nogolden_deal_scatter"), deal="scatter"),
+    dict(U.case("15d_fusion2", 2, 8, 7, 5, n=101, m=90, name="deal_last"), deal="last"),
+    dict(U.case("15d_sparse", 1, 8, 7, 5, n=101, m=90, name="deal_scatter"), deal="scatter"),
     # 16 x 16 with one nonzero per row on 4 ranks: null blocks and empty CSR blocks
-    U.case("15d_fusion1", 1, 4, 4, 1, name="nogolden_tiny_fusion1"),
-    U.case("15d_fusion2", 2, 4, 4, 1, name="nogolden_tiny_fusion2"),
-    U.case("15d_sparse", 4, 4, 4, 1, name="nogolden_tiny_sparse"),
-    U.case("25d_dense_replicate", 1, 4, 4, 1, name="nogolden_tiny_25d_dense"),
-    U.case("25d_sparse_replicate", 1, 4, 4, 1, name="nogolden_tiny_25d_sparse"),
-    U.case("15d_fusion1", 1, 8, 7, 5, n=100, m=61, name="nogolden_rect_fusion1"),
-    U.case("25d_dense_replicate", 1, 8, 7, 5, n=90, m=128, name="nogolden_rect_25d_dense"),
-    U.case("25d_sparse_replicate", 1, 8, 7, 5, n=128, m=77, name="nogolden_rect_25d_sparse"),
+    U.case("15d_fusion1", 1, 4, 4, 1, name="tiny_fusion1"),
+    U.case("15d_fusion2", 2, 4, 4, 1, name="tiny_fusion2"),
+    U.case("15d_sparse", 4, 4, 4, 1, name="tiny_sparse"),
+    U.case("25d_dense_replicate", 1, 4, 4, 1, name="tiny_25d_dense"),
+    U.case("25d_sparse_replicate", 1, 4, 4, 1, name="tiny_25d_sparse"),
+    U.case("15d_fusion1", 1, 8, 7, 5, n=100, m=61, name="rect_fusion1"),
+    U.case("25d_dense_replicate", 1, 8, 7, 5, n=90, m=128, name="rect_25d_dense"),
+    U.case("25d_sparse_replicate", 1, 8, 7, 5, n=128, m=77, name="rect_25d_sparse"),
 ]
 # the grid shapes of the 8-GPU runs (BASELINE.json configs 2-5): p=8 with c = 1, 2, 4, 8; 2.5D with s=2, c=2
 CASES_8 = [
@@ -59,12 +59,7 @@ CASES_8 = [
 def test_setup_path_matches_reference_rank_by_rank(nproc, cases):
     cases = [dict(c, script=[]) for c in cases]
     got = U.run_cases(nproc, cases, "gloo")
-    checked = 0
     for c in cases:
         want, src = U.reference_for(dict(c, script=[]), nproc)
-        if want is None:
-            continue
+        assert want is not None, f"no reference for {c['name']} (p={nproc}): run scripts/make_golden.py"
         U.compare_layout(got[c["name"]], want, c["alg"])
-        checked += 1
-    if checked == 0:
-        pytest.skip("neither oracle/_ref nor golden files available")

@@ -1,5 +1,5 @@
 """Multi-rank parity ON THE GPU against the REFERENCE's own code (oracle/_ref, or the committed
-golden files generated from it): every public operation of every algorithm, rank by rank --
+golden files generated from it by scripts/make_golden.py): every public operation of every algorithm, rank by rank --
 local value order bit-exact, fp64 outputs within 1e-11 relative (contract: 1e-5).
 
 How the ranks are mapped: with at least `nproc` GPUs each rank gets its own GPU and the ring
@@ -13,6 +13,7 @@ import numpy as np
 import pytest
 import torch
 
+from tests import golden_util as G
 from tests import mp_util as U
 
 pytestmark = pytest.mark.gpu
@@ -22,16 +23,16 @@ CASES = {
         U.case("15d_fusion2", 2, 8, 7, 5), U.case("15d_sparse", 1, 8, 7, 5), U.case("15d_sparse", 2, 8, 7, 5),
         U.case("25d_sparse_replicate", 2, 8, 7, 5),
         U.case("15d_fusion2", 1, 8, 7, 5, n=101), U.case("15d_sparse", 1, 8, 7, 5, n=101),  # padded trailing blocks
-        # wide factors (the r = 128 kernels); too large for a golden file: needs oracle/_ref
-        U.case("15d_fusion2", 1, 128, 9, 6, name="nogolden_fusion2_r128"),
-        U.case("15d_fusion1", 1, 128, 9, 6, name="nogolden_fusion1_r128")],
+        # wide factors (the r = 128 kernels)
+        U.case("15d_fusion2", 1, 128, 9, 6, name="fusion2_r128"),
+        U.case("15d_fusion1", 1, 128, 9, 6, name="fusion1_r128")],
     4: [U.case("15d_fusion1", 2, 8, 7, 5), dict(U.case("15d_fusion2", 1, 16, 7, 5), als=1), U.case("15d_fusion2", 4, 8, 7, 5),
         U.case("15d_sparse", 1, 8, 7, 5), dict(U.case("15d_sparse", 2, 32, 7, 5), als=1), dict(U.case("25d_dense_replicate", 1, 8, 7, 5), als=1),
         U.case("25d_sparse_replicate", 1, 8, 7, 5),
         U.case("15d_fusion1", 2, 8, 7, 5, n=99), U.case("25d_dense_replicate", 1, 8, 7, 5, n=99)],
     8: [U.case("15d_fusion1", 2, 8, 8, 5), U.case("15d_fusion2", 1, 8, 8, 5), U.case("15d_sparse", 1, 32, 8, 5),
         U.case("25d_dense_replicate", 2, 8, 8, 5), U.case("25d_sparse_replicate", 2, 8, 8, 5),
-        U.case("15d_fusion2", 2, 128, 10, 6, name="nogolden_fusion2_r128_p8")],
+        U.case("15d_fusion2", 2, 128, 10, 6, name="fusion2_r128_p8")],
 }
 
 
@@ -41,15 +42,12 @@ def transport_for(nproc):
 
 @pytest.mark.parametrize("nproc", [2, 4, 8])
 def test_all_operations_match_reference(nproc):
-    if nproc == 8 and torch.cuda.device_count() < 8:
-        pytest.skip("8 ranks only on an 8-GPU box (kept short on one GPU)")
     cases = CASES[nproc]
     got = U.run_cases(nproc, cases, transport_for(nproc), timeout=900)
     checked, worst = 0, 0.0
     for c in cases:
         want, src = U.reference_for(c, nproc)
-        if want is None:
-            continue
+        assert want is not None, f"no reference for {c['name']} (p={nproc}): run scripts/make_golden.py"
         try:
             U.compare_layout(got[c["name"]], want, c["alg"])
             worst = max(worst, U.compare_ops(got[c["name"]], want, c["script"]))
@@ -82,23 +80,29 @@ def test_gat_forward_matches_reference(nproc):
     """GAT forward pass (include/hnh/gat.hpp) rank by rank against the reference's gat.hpp run by oracle/_ref --
     including the fusion-2, c > 1 case where the reference's SpMM pass accumulates onto the gathered
     projection (15D_dense_shift.hpp:306-314 with initial_replicate = false)."""
-    from oracle import hnh_oracle as orc
-    from oracle import ref
-    from tests.mp_worker import gat_inputs
-    if not ref.available():
-        pytest.skip("oracle/_ref is not built")
     cases = GAT_CASES[nproc]
     got = U.run_cases(nproc, cases, transport_for(nproc), timeout=900)
     for c in cases:
+        want, _ = gat_reference(c, nproc)
+        for r in range(nproc):
+            have, w = got[c["name"]][r]["gat_out"], want[f"r{r}_gat_out"]
+            assert have.shape == tuple(w.shape), (c["name"], r, have.shape, w.shape)
+            err = G.rel_err(have, w)
+            assert err < 1e-11, (c["name"], r, err)
+
+
+def gat_reference(c, nproc):
+    """Every rank's GAT output of the reference's gat.hpp (oracle/_ref, or its golden file)."""
+    def compute():
+        from oracle import hnh_oracle as orc
+        from oracle import ref
+        from tests.mp_worker import gat_inputs
         N = 1 << c["logM"]
         rows, cols, _ = orc.er_tuples(c["logM"], c["npr"], c["seed"])
         layers, X0, weights = gat_inputs(N, c["gat"]["layers"], c["seed"])
         _, per_rank = ref.gat(c["alg"], nproc, c["c"], N, rows, cols, np.ones(len(rows)), layers, weights, c["gat"]["alpha"], X0)
-        for r, (want, _) in enumerate(per_rank):
-            have = got[c["name"]][r]["gat_out"]
-            assert have.shape == want.shape, (c["name"], r, have.shape, want.shape)
-            err = np.abs(have - want).max() / max(np.abs(want).max(), 1e-300)
-            assert err < 1e-11, (c["name"], r, err)
+        return {f"r{r}_gat_out": out for r, (out, _) in enumerate(per_rank)}
+    return U.reference_arrays(f"{c['name']}_p{nproc}", compute)
 
 
 HOSTPIPE_CASES = {
@@ -142,34 +146,43 @@ def test_als_cg_matches_reference_als(nproc):
     truth and starting embeddings, against the reference's own Distributed_ALS / cg_optimizer run by oracle/_ref --
     residuals and every rank's local embeddings.  Tolerance 1e-7 relative (contract 1e-5): 20 CG iterations separate
     the two summation orders."""
-    from oracle import hnh_oracle as orc
-    from oracle import ref
-    from tests.mp_worker import als_inputs
-    if not ref.available():
-        pytest.skip("oracle/_ref is not built")
     cases = ALS_CASES[nproc]
     got = U.run_cases(nproc, cases, transport_for(nproc), timeout=900)
     for c in cases:
+        want, _ = als_reference(c, nproc)
+        for r in range(nproc):
+            g = got[c["name"]][r]
+            assert np.allclose(g["als_res"], want["residual"], rtol=1e-7, atol=0), (c["name"], r, g["als_res"], want["residual"])
+            for have, w in ((g["als_A"], want[f"r{r}_A"]), (g["als_B"], want[f"r{r}_B"])):
+                assert have.shape == tuple(w.shape), (c["name"], r)
+                assert G.abs_err(have, w) <= 1e-7 * G.absmax(w), (c["name"], r)
+
+
+def als_reference(c, nproc):
+    """Residuals and every rank's local embeddings of the reference's Distributed_ALS (oracle/_ref, or its golden file)."""
+    def compute():
+        from oracle import hnh_oracle as orc
+        from oracle import ref
+        from tests.mp_worker import als_inputs
         N = 1 << c["logM"]
         rows, cols, _ = orc.er_tuples(c["logM"], c["npr"], c["seed"])
         want = ref.als(c["alg"], nproc, c["c"], c["R"], N, rows, cols, *als_inputs(N, c["R"], c["seed"]), 1, 10)
+        out = {"residual": np.asarray(want["residual"])}
         for r, (wA, wB) in enumerate(want["ranks"]):
-            g = got[c["name"]][r]
-            assert np.allclose(g["als_res"], want["residual"], rtol=1e-7, atol=0), (c["name"], r, g["als_res"], want["residual"])
-            for have, w in ((g["als_A"], wA), (g["als_B"], wB)):
-                assert have.shape == w.shape, (c["name"], r)
-                assert np.abs(have - w).max() <= 1e-7 * np.abs(w).max(), (c["name"], r)
+            out[f"r{r}_A"], out[f"r{r}_B"] = wA, wB
+        return out
+    return U.reference_arrays(f"{c['name']}_p{nproc}", compute)
 
 
 RECT_CASES = {
-    2: [U.case("15d_fusion2", 1, 8, 7, 5, n=120, m=75, name="nogolden_rect_fusion2"),
-        U.case("15d_fusion1", 2, 8, 7, 5, n=70, m=128, name="nogolden_rect_fusion1"),
-        U.case("15d_sparse", 2, 8, 7, 5, n=70, m=128, name="nogolden_rect_sparse")],
-    4: [U.case("15d_fusion1", 1, 8, 7, 5, n=100, m=61, name="nogolden_rect_fusion1"),
-        U.case("15d_fusion2", 2, 8, 7, 5, n=128, m=77, name="nogolden_rect_fusion2"),
-        U.case("15d_sparse", 1, 8, 7, 5, n=100, m=61, name="nogolden_rect_sparse"),
-        U.case("25d_dense_replicate", 1, 8, 7, 5, n=90, m=128, name="nogolden_rect_25d_dense"),
-        U.case("25d_sparse_replicate", 1, 8, 7, 5, n=128, m=77, name="nogolden_rect_25d_sparse")],
+    2: [U.case("15d_fusion2", 1, 8, 7, 5, n=120, m=75, name="rect_fusion2"),
+        U.case("15d_fusion1", 2, 8, 7, 5, n=70, m=128, name="rect_fusion1"),
+        U.case("15d_sparse", 2, 8, 7, 5, n=70, m=128, name="rect_sparse")],
+    4: [U.case("15d_fusion1", 1, 8, 7, 5, n=100, m=61, name="rect_fusion1"),
+        U.case("15d_fusion2", 2, 8, 7, 5, n=128, m=77, name="rect_fusion2"),
+        U.case("15d_sparse", 1, 8, 7, 5, n=100, m=61, name="rect_sparse"),
+        U.case("25d_dense_replicate", 1, 8, 7, 5, n=90, m=128, name="rect_25d_dense"),
+        U.case("25d_sparse_replicate", 1, 8, 7, 5, n=128, m=77, name="rect_25d_sparse")],
 }
 
 
@@ -177,9 +190,6 @@ RECT_CASES = {
 def test_rectangular_matrices_match_reference(nproc):
     """M != N (more columns than rows and the reverse, sizes that do not divide evenly): every public operation of
     every algorithm against the reference's own code, as in test_all_operations_match_reference."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref is not built")
     cases = RECT_CASES[nproc]
     got = U.run_cases(nproc, cases, transport_for(nproc), timeout=900)
     for c in cases:
@@ -191,19 +201,16 @@ def test_rectangular_matrices_match_reference(nproc):
             raise AssertionError(f"case {c['name']} (p={nproc}, reference from {src}): {e}") from e
 
 
-TINY_CASES = [U.case("15d_fusion1", 1, 4, 4, 1, name="nogolden_tiny_fusion1"), U.case("15d_fusion2", 2, 4, 4, 1, name="nogolden_tiny_fusion2"),
-              U.case("15d_fusion2", 1, 4, 4, 1, name="nogolden_tiny_fusion2_c1"), U.case("15d_sparse", 4, 4, 4, 1, name="nogolden_tiny_sparse"),
-              U.case("15d_sparse", 1, 4, 4, 1, name="nogolden_tiny_sparse_c1"),
-              U.case("25d_dense_replicate", 1, 4, 4, 1, name="nogolden_tiny_25d_dense"),
-              U.case("25d_sparse_replicate", 1, 4, 4, 1, name="nogolden_tiny_25d_sparse")]
+TINY_CASES = [U.case("15d_fusion1", 1, 4, 4, 1, name="tiny_fusion1"), U.case("15d_fusion2", 2, 4, 4, 1, name="tiny_fusion2"),
+              U.case("15d_fusion2", 1, 4, 4, 1, name="tiny_fusion2_c1"), U.case("15d_sparse", 4, 4, 4, 1, name="tiny_sparse"),
+              U.case("15d_sparse", 1, 4, 4, 1, name="tiny_sparse_c1"),
+              U.case("25d_dense_replicate", 1, 4, 4, 1, name="tiny_25d_dense"),
+              U.case("25d_sparse_replicate", 1, 4, 4, 1, name="tiny_25d_sparse")]
 
 
 def test_null_and_empty_blocks_match_reference():
     """A 16 x 16 matrix with one nonzero per row on 4 ranks: most blocks are null or empty (the reference skips them,
     sparse_kernels.cpp:25-27,71-73,85-87); every operation must still agree with it."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref is not built")
     got = U.run_cases(4, TINY_CASES, transport_for(4), timeout=900)
     for c in TINY_CASES:
         want, src = U.reference_for(c, 4)
@@ -234,8 +241,7 @@ def test_device_side_setup_matches_reference(nproc):
     checked = 0
     for c in cases:
         want, src = U.reference_for(c, nproc)
-        if want is None:
-            continue
+        assert want is not None, f"no reference for {c['name']} (p={nproc}): run scripts/make_golden.py"
         info = json.loads(str(got[c["name"]][0]["setup_times"]))
         assert any("(device)" in k for k in info), (c["name"], "the device setup path did not run", info)
         try:
@@ -255,8 +261,7 @@ def test_peer_ring_failure_on_one_rank_is_a_collective_fallback():
     got = U.run_cases(2, cases, transport_for(2), timeout=600, env_extra={"HNH_TEST_PEERRING_FAIL": "1"})
     for c in cases:
         want, src = U.reference_for(c, 2)
-        if want is None:
-            pytest.skip("neither oracle/_ref nor golden files available")
+        assert want is not None, f"no reference for {c['name']}: run scripts/make_golden.py"
         U.compare_layout(got[c["name"]], want, c["alg"])
         U.compare_ops(got[c["name"]], want, c["script"])
         for rank_out in got[c["name"]]:
