@@ -42,6 +42,10 @@ ABI = {
     "hnh_leaky_relu_f64": (C.c_int, [_P, _P, _I64, C.c_double, _P]),
     "hnh_relu_cols_f64": (C.c_int, [_P, _I64, _I64, _P, _I64, _I64, _P]),
     "hnh_dgemm_f64": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _P]),
+    "hnh_relu_cols_backward_f64": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _I64, _P]),
+    "hnh_leaky_relu_slope_f64": (C.c_int, [_P, _P, _I64, C.c_double, _P]),
+    "hnh_dgemm_tn_f64": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _P]),
+    "hnh_dgemm_nt_f64": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, C.c_double, _P]),
     "hnh_block_create_host": (C.c_int, [_P, _P, _I64, _I64, _I64, C.c_int, C.POINTER(_P)]),
     "hnh_block_destroy": (None, [_P]),
     "hnh_block_run_host": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, C.c_int, C.c_int, _P]),
@@ -182,6 +186,12 @@ ABI.update({
     "hnhd_gat_set_input": (C.c_int, [_P, _P]),
     "hnhd_gat_get_buffer": (C.c_int, [_P, C.c_int, _P]),
     "hnhd_gat_forward": (C.c_int, [_P]),
+    "hnhd_gat_supports_backward": (C.c_int, [_P]),
+    "hnhd_gat_backward": (C.c_int, [_P, _P]),
+    "hnhd_gat_get_weight_grad": (C.c_int, [_P, C.c_int, C.c_int, _P]),
+    "hnhd_gat_get_input_grad": (C.c_int, [_P, _P]),
+    "hnhd_gat_get_weight": (C.c_int, [_P, C.c_int, C.c_int, _P]),
+    "hnhd_gat_sgd_step": (C.c_int, [_P, C.c_double]),
     "hnhd_gat_destroy": (None, [_P]),
     "hnhd_timer_start": (C.c_int, []),
     "hnhd_timer_stop": (C.c_int, [C.POINTER(C.c_double)]),

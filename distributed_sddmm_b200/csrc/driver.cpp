@@ -462,6 +462,50 @@ int hnhd_gat_forward(hnhd_gat_t *g) {
         g->g->forwardPass();
     });
 }
+int hnhd_gat_supports_backward(hnhd_gat_t *g) {
+    if (!g) return hnh::set_error(HNH_E_INVALID, "null gat");
+    return g->g->supportsBackward() ? 1 : 0;
+}
+int hnhd_gat_backward(hnhd_gat_t *g, const double *host_output_grad) {
+    return guarded([&] {
+        if (!g || !host_output_grad) throw hnh::Error(HNH_E_INVALID, "hnhd_gat_backward: null argument");
+        GAT &net = *g->g;
+        const string why = net.backwardUnsupportedReason();  // refuse before touching the device
+        if (!why.empty()) throw hnh::Error(HNH_E_INVALID, "GAT::backwardPass: " + why);
+        DenseMatrix grad(net.buffers.back().rows(), net.buffers.back().cols());
+        grad.copy_from_host(host_output_grad);
+        net.backwardPass(grad);
+    });
+}
+int hnhd_gat_get_weight_grad(hnhd_gat_t *g, int layer, int head, double *host) {
+    return guarded([&] {
+        if (!host) throw hnh::Error(HNH_E_INVALID, "null host pointer");
+        gat_weight(g, layer, head);  // validates layer and head
+        if (g->g->wGrads.size() != g->g->layers.size())
+            throw hnh::Error(HNH_E_INVALID, "hnhd_gat_get_weight_grad: no gradients (run hnhd_gat_backward first)");
+        g->g->wGrads[(size_t)layer][(size_t)head].copy_to_host(host);
+    });
+}
+int hnhd_gat_get_input_grad(hnhd_gat_t *g, double *host) {
+    return guarded([&] {
+        if (!g || !host) throw hnh::Error(HNH_E_INVALID, "hnhd_gat_get_input_grad: null argument");
+        if (g->g->input_grad.size() != g->g->buffers[0].size())
+            throw hnh::Error(HNH_E_INVALID, "hnhd_gat_get_input_grad: no gradients (run hnhd_gat_backward first)");
+        g->g->input_grad.copy_to_host(host);
+    });
+}
+int hnhd_gat_get_weight(hnhd_gat_t *g, int layer, int head, double *host) {
+    return guarded([&] {
+        if (!host) throw hnh::Error(HNH_E_INVALID, "null host pointer");
+        gat_weight(g, layer, head).copy_to_host(host);
+    });
+}
+int hnhd_gat_sgd_step(hnhd_gat_t *g, double lr) {
+    return guarded([&] {
+        if (!g) throw hnh::Error(HNH_E_INVALID, "null gat");
+        g->g->applyGradients(lr);
+    });
+}
 void hnhd_gat_destroy(hnhd_gat_t *g) { delete g; }
 
 }  // extern "C"

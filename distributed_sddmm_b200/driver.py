@@ -338,8 +338,8 @@ def benchmark_algorithm(S: SpmatLocal, name: str, R: int, c: int, fused=True, ap
 
 
 class GAT:
-    """Multi-head graph attention forward pass (include/hnh/gat.hpp).  layers: [(input_features,
-    features_per_head, num_heads), ...].  The algorithm object must outlive this one."""
+    """Multi-head graph attention (include/hnh/gat.hpp): forward pass, backward pass and a plain SGD step.
+    layers: [(input_features, features_per_head, num_heads), ...].  The algorithm object must outlive this one."""
 
     def __init__(self, alg: Algorithm, layers, leaky_relu_alpha: float = 0.2):
         self.alg = alg
@@ -375,6 +375,39 @@ class GAT:
 
     def forward(self):
         check(lib().hnhd_gat_forward(self.h), "gat_forward")
+
+    def supports_backward(self) -> bool:
+        rc = lib().hnhd_gat_supports_backward(self.h)
+        if rc < 0:
+            check(rc, "gat_supports_backward")
+        return rc == 1
+
+    def backward(self, grad):
+        """Gradients of L from grad = dL/d(output of the last layer) (this rank's rows), after forward() with the
+        current weights.  Collective over the ranks; overwrites the gradients."""
+        grad = np.ascontiguousarray(grad, dtype=np.float64)
+        want = self.buffer_shape(len(self.layers))
+        assert grad.shape == want, (grad.shape, want)
+        check(lib().hnhd_gat_backward(self.h, grad.ctypes.data), "gat_backward")
+
+    def weight_grad(self, layer: int, head: int):
+        out = np.empty(self.weight_shape(layer, head), dtype=np.float64)
+        check(lib().hnhd_gat_get_weight_grad(self.h, layer, head, out.ctypes.data), "gat_get_weight_grad")
+        return out
+
+    def input_grad(self):
+        out = np.empty(self.buffer_shape(0), dtype=np.float64)
+        check(lib().hnhd_gat_get_input_grad(self.h, out.ctypes.data), "gat_get_input_grad")
+        return out
+
+    def weight(self, layer: int, head: int):
+        out = np.empty(self.weight_shape(layer, head), dtype=np.float64)
+        check(lib().hnhd_gat_get_weight(self.h, layer, head, out.ctypes.data), "gat_get_weight")
+        return out
+
+    def sgd_step(self, lr: float):
+        """W -= lr * W_grad for every weight (after backward())."""
+        check(lib().hnhd_gat_sgd_step(self.h, float(lr)), "gat_sgd_step")
 
     def __del__(self):
         try:

@@ -157,6 +157,21 @@ int hnh_relu_cols_f64(double *dst, int64_t ld_dst, int64_t col0, const double *s
 int hnh_dgemm_f64(double *C, const double *A, const double *B, int64_t m, int64_t n, int64_t k,
                   void *stream);
 
+/* ---- GAT backward pass helpers (include/hnh/gat.hpp, GAT::backwardPass) ----------------------
+ * dst[i, j] = grad[i, col0 + j] if out[i, col0 + j] > 0, else 0 (ReLU'(0) = 0): the gradient of a head's
+ * column window.  grad and out have ld columns, dst is rows x cols, contiguous. */
+int hnh_relu_cols_backward_f64(double *dst, const double *grad, const double *out, int64_t ld, int64_t col0,
+                               int64_t rows, int64_t cols, void *stream);
+/* dst[i] = 1 if src[i] > 0, else alpha: the derivative of hnh_leaky_relu_f64 (alpha at 0; dst may alias src) */
+int hnh_leaky_relu_slope_f64(double *dst, const double *src, int64_t n, double alpha, void *stream);
+/* C (k x n) = A^T B for A (m x k) and B (m x n), row-major; m (the graph rows) is the long dimension.  DMMA tiles over
+ * row chunks, partial tiles summed in a fixed order: deterministic, repeated calls agree bit for bit.  m == 0 gives
+ * C = 0.  Allocates its scratch stream-ordered. */
+int hnh_dgemm_tn_f64(double *C, const double *A, const double *B, int64_t m, int64_t n, int64_t k, void *stream);
+/* C (m x n) = A B^T + beta * C for A (m x k) and B (n x k), row-major; beta is 0 or 1 (HNH_E_INVALID otherwise). */
+int hnh_dgemm_nt_f64(double *C, const double *A, const double *B, int64_t m, int64_t n, int64_t k, double beta,
+                     void *stream);
+
 /* ---- host-side setup helpers (untimed; HOST pointers) --------------------------------------
  * hnh_er_generate_host replaces the CombBLAS Graph500 generator call of
  * SpmatLocal::loadTuples(false, logM, nnz_per_row) (SpmatLocal.hpp:499-516): rows

@@ -178,7 +178,7 @@ int hnhd_als_run(hnhd_alg_t *alg, const double *hostAgt, const double *hostBgt, 
                  const double *hostB0, int steps, int cg_iters, double *out2, double *hostA_out,
                  double *hostB_out);
 
-/* ---- GAT forward pass (include/hnh/gat.hpp; reference gat.hpp:26-113) -----------------------
+/* ---- GAT (include/hnh/gat.hpp; reference gat.hpp:26-113) ------------------------------------
  * layers3: n_layers triples (input_features, features_per_head, num_heads).  The object keeps a
  * pointer to `alg`, which must outlive it.  buffer 0 is the network input, buffer i + 1 the output
  * of layer i; weights are input_width x head_width, row-major, as hnhd_gat_weight_shape reports. */
@@ -191,6 +191,16 @@ int hnhd_gat_buffer_shape(hnhd_gat_t *g, int buffer, int64_t *rows, int64_t *col
 int hnhd_gat_set_input(hnhd_gat_t *g, const double *host);          /* buffer 0 */
 int hnhd_gat_get_buffer(hnhd_gat_t *g, int buffer, double *host);   /* synchronises */
 int hnhd_gat_forward(hnhd_gat_t *g);                                /* forwardPass(); stream-ordered */
+/* Backward pass (GAT::backwardPass) from dL/d(last buffer) = host_output_grad (this rank's rows, the shape of the last
+ * buffer).  Needs the forward pass of the current weights in the buffers; overwrites the gradients.  Collective: the
+ * weight gradients are summed over all ranks.  HNH_E_INVALID, with nothing enqueued, where
+ * hnhd_gat_supports_backward() is 0; the error string says why. */
+int hnhd_gat_supports_backward(hnhd_gat_t *g);                      /* 1, 0, or a negative code */
+int hnhd_gat_backward(hnhd_gat_t *g, const double *host_output_grad);
+int hnhd_gat_get_weight_grad(hnhd_gat_t *g, int layer, int head, double *host); /* weight shape; synchronises */
+int hnhd_gat_get_input_grad(hnhd_gat_t *g, double *host);           /* shape of buffer 0; synchronises */
+int hnhd_gat_get_weight(hnhd_gat_t *g, int layer, int head, double *host);      /* synchronises */
+int hnhd_gat_sgd_step(hnhd_gat_t *g, double lr);                    /* W -= lr * W_grad for every weight */
 void hnhd_gat_destroy(hnhd_gat_t *g);
 
 #ifdef __cplusplus
